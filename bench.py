@@ -6,6 +6,12 @@ model (configs[3]), at 1/2/4/8 GPUs; configs[4] (8 GiB, vocab 100000) with --con
     python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (GPU)
     python bench.py --impl reference [...]                         the reference's own CPU code, bounded sample
 
+Every timed leg runs exactly K timed steps. --dump-outputs DIR: after the timed steps, rank 0 writes what each timed leg
+computed in its last step as DIR/<name>.npy in float64 (exact for ids, counts and bytes): train_merges, train_counts,
+train_<other mode>_merges / _counts, encode_ids (the ids of the last encode batch), decode_bytes, config5_merges. An
+array of more than DUMP_ROWS rows is cut to a fixed, seeded sample of its rows, kept in order. The inputs depend on the
+arguments alone (seeded generators), so two builds can be compared file by file.
+
 One JSON line on stdout (rank 0). PyTorch is plumbing only: torch.distributed (NCCL) barrier / max over ranks, device
 buffers, streams and events. All compute goes through the C ABI of libminbpe_b200.so (include/minbpe_b200.h).
 
@@ -32,11 +38,28 @@ import tempfile
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
-SEED_TRAIN, SEED_ENCODE, SEED_CONFIG5 = 0x5EED0001, 0x5EED0002, 0x5EED0003
+SEED_TRAIN, SEED_ENCODE, SEED_CONFIG5, SEED_DUMP = 0x5EED0001, 0x5EED0002, 0x5EED0003, 0x5EED00D0
 MIB = 1 << 20
+DUMP_ROWS = 1 << 19  # per array: the seven arrays of --dump-outputs stay under 64 MiB in float64
+
+
+def dump_rows(n):
+    """indices of the rows --dump-outputs keeps of an n-row array: all of them, or a fixed seeded sample in order"""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(SEED_DUMP).choice(n, DUMP_ROWS, replace=False))
+
+
+def write_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, x in arrays.items():
+        x = np.asarray(x)
+        np.save(os.path.join(d, name + ".npy"), x[dump_rows(len(x))].astype(np.float64))
 
 
 def load_pkg():
@@ -93,6 +116,7 @@ class ClockSampler:
         if not self.proc:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         self.proc.terminate()
+        self.proc.wait()
         sm, mx, reasons = [], None, set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         for t, line in self.rows:
@@ -207,8 +231,10 @@ def run_reference_arm(a, rank):
         return
     vals = []
     for _ in range(a.warmup + a.steps):
-        cb, _, _ = ref_train_sample(a.ref_sample_mib, a.ref_merges, a.mode, a.corpus_mib * MIB)
+        cb, merges, _ = ref_train_sample(a.ref_sample_mib, a.ref_merges, a.mode, a.corpus_mib * MIB)
         vals.append(cb)
+    if a.dump_outputs:
+        write_outputs(a.dump_outputs, {"train_merges": merges})
     vals = vals[a.warmup:] or vals
     v = sum(x["value"] for x in vals) / len(vals)
     cb = dict(vals[-1], value=v)
@@ -250,7 +276,6 @@ def main():
     ap.add_argument("--ref-sample-mib", type=int, default=4)
     ap.add_argument("--ref-merges", type=int, default=128)
     ap.add_argument("--ref-encode-mib", type=int, default=256)
-    ap.add_argument("--e2e-budget-s", type=float, default=60.0)
     ap.add_argument("--skip-encode", action="store_true")
     ap.add_argument("--skip-first", action="store_true", help="skip the first-occurrence-mode train line")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
@@ -259,7 +284,10 @@ def main():
     ap.add_argument("--config5-vocab", type=int, default=100000)
     ap.add_argument("--selftest", action="store_true", help="N > 1: diff the sharded trainer against the oracle on the goldens first")
     ap.add_argument("--no-check", action="store_true", help="skip the full-size diff of the merge list against the CPU oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of every leg as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -268,7 +296,6 @@ def main():
         run_reference_arm(a, rank)
         return
 
-    import numpy as np
     import torch
     import torch.distributed as dist
 
@@ -370,6 +397,7 @@ def main():
         ms_per_step, (merges, counts, stats) = timed_steps(lambda: strainer.run(a.vocab, a.mode, stream), a.warmup, a.steps)
         what = (f"mbpe_sharded_trainer_run over {world} GPUs: unique chunks sharded (resident), replicated pair table, "
                 "per-merge exchange of count deltas over NVLink")
+    dumps = {"train_merges": merges, "train_counts": counts}
     n_done = len(merges)
     value = n_done / (ms_per_step / 1e3)
     model_sha = hashlib.sha256(merges.tobytes()).hexdigest()
@@ -413,16 +441,14 @@ def main():
     if world == 1:
         text_pinned = torch.empty(len(text), dtype=torch.uint8, pin_memory=True)  # the step's input, in pinned host memory
         text_pinned.numpy()[:] = text
-        e2e_times, t_budget = [], time.time()
-        for i in range(1 + max(1, a.steps)):  # the first call is a warm-up: it sizes the tokenizer's resident device buffers
+        e2e_times = []
+        for i in range(1 + a.steps):  # the first call is a warm-up: it sizes the tokenizer's resident device buffers
             barrier()
             t0 = time.time()
             tk.train(text_pinned.numpy(), a.vocab, a.mode)
             torch.cuda.synchronize()
             if i:
                 e2e_times.append(time.time() - t0)
-            if time.time() - t_budget > a.e2e_budget_s and e2e_times:
-                break
         e2e_s = sum(e2e_times) / len(e2e_times)
         st2 = tk.last_train_stats()
         assert hashlib.sha256(tk.merges().tobytes()).hexdigest() == model_sha, "tokenizer path and trainer path disagree"
@@ -446,7 +472,7 @@ def main():
     else:
         # N > 1: the C-ABI call with HOST buffers -- every rank uploads its shard of the unique chunks inside the call
         e2e_times = []
-        for i in range(1 + max(1, min(a.steps, 2))):
+        for i in range(1 + a.steps):
             barrier()
             t0 = time.time()
             sm, sc, sst = comm.train(tok, off, w, a.vocab, a.mode, stream)
@@ -482,9 +508,10 @@ def main():
     if not a.skip_first:
         other = "first" if a.mode == "lexical" else "lexical"
         if world == 1:
-            o_ms, (o_m, o_c, o_st) = timed_steps(lambda: trainer.run(a.vocab, other, a.engine, stream), 1, max(1, min(a.steps, 2)))
+            o_ms, (o_m, o_c, o_st) = timed_steps(lambda: trainer.run(a.vocab, other, a.engine, stream), 1, a.steps)
         else:
-            o_ms, (o_m, o_c, o_st) = timed_steps(lambda: strainer.run(a.vocab, other, stream), 1, max(1, min(a.steps, 2)))
+            o_ms, (o_m, o_c, o_st) = timed_steps(lambda: strainer.run(a.vocab, other, stream), 1, a.steps)
+        dumps.update({f"train_{other}_merges": o_m, f"train_{other}_counts": o_c})
         leg = {"mode": other, "value": len(o_m) / (o_ms / 1e3), "unit": "merges/s", "ms_per_step": o_ms, "merges": int(len(o_m)),
                "merges_sha256": hashlib.sha256(o_m.tobytes()).hexdigest()}
         if not a.no_check and rank == 0:
@@ -494,7 +521,7 @@ def main():
             leg["oracle_check"] = {"merges_equal": bool(om.shape == o_m.shape and (om == o_m).all()),
                                    "counts_equal": bool(oc.shape == o_c.shape and (oc == o_c).all()), "oracle_s": time.time() - t0}
         line["train_" + other] = leg
-        line["gpu_launches"] += int(o_st["n_launches"]) * max(1, min(a.steps, 2))
+        line["gpu_launches"] += int(o_st["n_launches"]) * a.steps
     if world == 1:
         trainer.close()
     else:
@@ -550,6 +577,8 @@ def main():
             e.close()
         # the same text again through the now-warm caches, for the record (not the headline: config 4 sees its text once)
         warm_ms, _ = timed_steps(lambda: encode_pass(enc), 1, n_steps)
+        if a.dump_outputs and rank == 0:  # the last timed step left the ids of the last batch in d_out
+            dumps["encode_ids"] = d_out[torch.from_numpy(dump_rows(int(d_n.item()))).to(dev)].cpu().numpy().view(np.uint32)
         # untimed: id counts of every batch for the algorithmic-byte figure; the first batch's ids are kept for the checks
         first_ids = None
         for bt in reversed(batches):
@@ -566,6 +595,8 @@ def main():
         dec_ms, _ = timed_steps(lambda: enc.decode_device(d_out.data_ptr(), bt0["n_ids"], d_txt.data_ptr(), bt0["n_bytes"] + 64,
                                                           d_ntxt.data_ptr(), stream), max(1, min(a.warmup, 3)), n_steps)
         n_txt = int(d_ntxt.item())
+        if a.dump_outputs and rank == 0:
+            dumps["decode_bytes"] = d_txt[torch.from_numpy(dump_rows(n_txt)).to(dev)].cpu().numpy()
         roundtrip = all_true(n_txt == bt0["n_bytes"] and bool(torch.equal(d_txt[:n_txt], bt0["d_bytes"])))
         b_dec = int(sum_over_ranks(4 * bt0["n_ids"] + n_txt))
         dec_bytes = int(sum_over_ranks(n_txt))
@@ -700,6 +731,7 @@ def main():
             leg5["same_merges_on_every_rank"] = all_true(bool((h == h0).all()))
         if err5 is None:
             line["config5"] = leg5
+            dumps["config5_merges"] = m5
         del pin5
 
     # ---------------- CPU baseline (rank 0, N == 1 only): the compiled reference on bounded samples --------------------
@@ -729,6 +761,8 @@ def main():
     if clocks:
         line["clocks"] = clocks.summary()
     if rank == 0:
+        if a.dump_outputs:
+            write_outputs(a.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
